@@ -229,6 +229,31 @@ def _ev_ms(fn, reps=1, warm=1):
     return e0.elapsed_time(e1) / reps
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each named tensor as `<out_dir>/<name>.npy`, float64 kept, every other dtype as float32, at most
+    DUMP_LIMIT_BYTES in all.  A tensor too large for its share of that limit is written as a fixed seeded sample of its
+    flattened elements (1-D): the positions depend only on its shape, so dumps of two builds compare element for
+    element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    budget = DUMP_LIMIT_BYTES - 1024 * len(items)        # room for the .npy headers
+    for i, (name, t) in enumerate(items):
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        share = budget // (len(items) - i)
+        n = share // dt.itemsize
+        if t.numel() > n:
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), size=n))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.detach().to("cpu", dt).numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        budget -= a.nbytes
+
+
 def parity_check(pipe, devin, dev, kw):
     """2 DDIM steps of the BENCHMARKED configuration (same weights, same inputs, graph replay as timed) against the fp32
     oracle and the stock bf16 torch execution on the same GPU.  Returns the dict stored under config.parity_check and
@@ -428,6 +453,8 @@ def run_product(args):
         torch.cuda.synchronize()
         torch.cuda.profiler.stop()
     barrier()
+    if args.dump_outputs and rank == 0:   # here: the calls below reuse the CUDA graph's output buffers
+        dump_outputs(args.dump_outputs, {"video": video, "latents": lat})
     t_dev = torch.tensor([e0.elapsed_time(e1) / 1e3], device=dev, dtype=torch.float64)
     launches = _lib.launch_count() - l0
     if pipe.use_cuda_graph:            # python-side calls happen once at capture; every replay re-launches them
@@ -637,8 +664,14 @@ def run_svd(args):
     sampler = ClockSampler(0)
     sampler.start()
     l0 = _lib.launch_count()
-    t_dev = _ev_ms(lambda: clip(devin), reps=args.steps, warm=0) / 1e3
+    last = []
+
+    def timed_clip():
+        last[:] = clip(devin)
+    t_dev = _ev_ms(timed_clip, reps=args.steps, warm=0) / 1e3
     launches = _lib.launch_count() - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"frames": torch.stack(last)})
 
     def e2e():
         inp = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
@@ -697,21 +730,22 @@ def run_vae(args):
         lat = torch.randn(1, 4, n, LAT, LAT, generator=g).to(dtype).to(dev)
         img = torch.randn(min(n, 64), 3, HW, HW, generator=g).clamp(-1, 1).to(dtype).to(dev)      # encoded in rounds of <= 64
         gather = torch.empty((world, n, HW, HW, 3), dtype=torch.uint8, device=dev) if world > 1 else None
+        outs = {}
 
         def decode():
             fr = vae.decode_frames_uint8(lat)
             if world > 1:
                 dist.all_gather_into_tensor(gather, fr.unsqueeze(0))
-            return fr
+            outs["frames"] = fr
 
         def encode():
             done = 0
             while done < n:
                 k = min(img.shape[0], n - done)
-                vae.encode(img[:k])
+                outs["latent_parameters"] = vae.encode(img[:k]).latent_dist.parameters
                 done += k
-        t_dec = torch.tensor([_ev_ms(decode, reps=1 if n_total >= 512 else 2, warm=1)], device=dev, dtype=torch.float64)
-        t_enc = torch.tensor([_ev_ms(encode, reps=1 if n_total >= 512 else 2, warm=1)], device=dev, dtype=torch.float64)
+        t_dec = torch.tensor([_ev_ms(decode, reps=args.steps, warm=args.warmup)], device=dev, dtype=torch.float64)
+        t_enc = torch.tensor([_ev_ms(encode, reps=args.steps, warm=args.warmup)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t_dec, op=dist.ReduceOp.MAX)
             dist.all_reduce(t_enc, op=dist.ReduceOp.MAX)
@@ -722,10 +756,13 @@ def run_vae(args):
                      "decode_frac_of_peak": d_fps * 2.515 / world / peak_tf, "encode_frac_of_peak": e_fps * 1.117 / world / peak_tf})
         del lat, img, gather
         torch.cuda.empty_cache()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
     if rank == 0:
         last = rows[-1]
         line = {"metric": "vae_decode_frames_per_sec_512x512", "value": last["decode_frames_per_s"], "unit": UNIT,
-                "n_gpus": world, "steps": 1, "warmup": 1, "ms_per_step": 1024 / last["decode_frames_per_s"] * 1e3,
+                "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
+                "ms_per_step": 1024 / last["decode_frames_per_s"] * 1e3,
                 "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
                 "config": {"workload": "config5: AutoencoderKL (SD VAE, random init) decode [N,4,64,64] -> uint8 512x512 frames and "
                                        "encode [N,3,512,512], N = 64..1024 split evenly over the GPUs, one all-gather of decoded frames",
@@ -758,7 +795,14 @@ def main():
     ap.add_argument("--workload", default="config2", choices=["config2", "svd", "vae"],
                     help="config2 (default, BASELINE's headline), svd (BASELINE config 4, 1 GPU) or vae (config 5: VAE-only "
                          "sweep, frames split over the GPUs); svd / vae exist for this repo's arm only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy, float32, "
+                         "64 MB at most (larger outputs as a fixed seeded sample); inputs and weights are seeded")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records this repo's arm; the reference arm times a bounded CPU sample only")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "svd":

@@ -226,7 +226,8 @@ def vae_fullsize_golden():
 def oddsize_unet_golden():
     """Verbatim reference UNet at a latent size that is NOT a multiple of 8 (15 x 17: what train.py:738-742 produces for
     most prompt images): exercises `forward_upsample_size` (models/unet_3d_condition_mask.py:377-383,486-491) and the odd
-    stride-2 convolutions.  SMALL config, fp16-rounded weights and inputs, fp32 math."""
+    stride-2 convolutions.  SMALL config, fp16-rounded weights and inputs, fp32 math; `out_f64` is the same forward in
+    float64, which a different CPU's convolution kernels reproduce far below the fp32 rounding of `out`."""
     from models.unet_3d_condition_mask import UNet3DConditionModel            # verbatim reference
     torch.manual_seed(0)
     ref = UNet3DConditionModel(**SMALL).eval()
@@ -239,8 +240,11 @@ def oddsize_unet_golden():
     with torch.no_grad():
         out = ref(inp["sample"], 321, inp["ehs"], condition_latent=inp["cond"], mask=inp["mask"],
                   motion=torch.tensor([5.0])).sample
+        i64 = {k: v.double() for k, v in inp.items()}
+        out_f64 = ref.double()(i64["sample"], 321, i64["ehs"], condition_latent=i64["cond"], mask=i64["mask"],
+                               motion=torch.tensor([5.0], dtype=torch.float64)).sample
     torch.save({"config": SMALL, "inputs": {k: v.half() for k, v in inp.items()}, "timestep": 321, "motion": 5.0,
-                "out": out}, os.path.join(HERE, "unet_small_oddsize_ref.pt"))
+                "out": out, "out_f64": out_f64}, os.path.join(HERE, "unet_small_oddsize_ref.pt"))
     print("unet_small_oddsize_ref.pt", tuple(out.shape), float(out.abs().mean()))
 
 
@@ -429,8 +433,32 @@ def forward_branches_golden():
           "| timestep_cond changes output by", float((out_tc - base).abs().mean()))
 
 
+def config_errors_golden():
+    """What the VERBATIM UNet3DConditionModel constructor (models/unet_3d_condition_mask.py:118-131) raises for each
+    inconsistent config of tests/test_unet_config_cpu.py: exception type and message, as JSON."""
+    import json
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_unet_config_cpu import BAD
+    from models.unet_3d_condition_mask import UNet3DConditionModel            # verbatim reference
+    cases = []
+    for cfg in BAD:
+        try:
+            UNet3DConditionModel(**cfg)
+            err = None
+        except Exception as e:
+            err = {"type": type(e).__name__, "message": str(e)}
+        cases.append({"config": cfg, "error": err})
+    with open(os.path.join(HERE, "unet_config_errors_ref.json"), "w") as f:
+        json.dump({"cases": cases}, f, indent=1)
+        f.write("\n")
+    print("unet_config_errors_ref.json:", [c["error"] and c["error"]["type"] for c in cases])
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "svd":
+    if len(sys.argv) > 1 and sys.argv[1] == "config_errors":
+        import diffusers  # noqa: F401  (the shim)
+        config_errors_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "svd":
         svd_goldens()
     elif len(sys.argv) > 1 and sys.argv[1] == "svd_text":
         import diffusers  # noqa: F401  (the shim)

@@ -1,8 +1,10 @@
 """Constructor behaviour of the UNet3DConditionModel mirror without a GPU: the three configuration checks of
-models/unet_3d_condition_mask.py:118-131 raise ValueError in the same cases as the verbatim reference class (checked where /root/reference exists), the config object
+models/unet_3d_condition_mask.py:118-131 raise the same ValueError as the verbatim reference class (whose outcome
+tests/golden/unet_config_errors_ref.json records: `python tests/golden/make_golden.py config_errors`), the config object
 exposes what callers read (train.py:91 `unet.config.in_channels`, models/pipeline.py:107 `unet.config.sample_size`),
 `conv_in.weight/bias` are nn.Parameters (train.py:98-101), and unknown block types are rejected
 (models/unet_3d_blocks.py:96,172)."""
+import json
 import os
 import sys
 
@@ -21,26 +23,22 @@ BAD = [
 ]
 
 
-def _verbatim_reference_class():
-    """The reference's own class over the diffusers shim -- only where /root/reference exists (the build container)."""
-    if not os.path.isdir("/root/reference/models"):
-        return None
-    sys.path.insert(0, os.path.join(os.path.dirname(HERE), "oracle", "shim"))
-    sys.path.insert(0, "/root/reference")
-    from models.unet_3d_condition_mask import UNet3DConditionModel as Ref
-    return Ref
+def _reference_outcome(i):
+    """What the reference's own class raised for BAD[i] (tests/golden/unet_config_errors_ref.json)."""
+    with open(os.path.join(HERE, "golden", "unet_config_errors_ref.json")) as f:
+        case = json.load(f)["cases"][i]
+    assert case["config"] == json.loads(json.dumps(BAD[i])), "fixture was generated from a different config"
+    return case["error"]
 
 
 @pytest.mark.parametrize("i", range(len(BAD)))
 def test_inconsistent_configs_raise_like_the_reference(i):
     from animate_anything_b200.unet_3d_condition_mask import UNet3DConditionModel
-    cfg = BAD[i]
-    ref = _verbatim_reference_class()
-    if ref is not None:
-        with pytest.raises(ValueError):
-            ref(**cfg)
-    with pytest.raises(ValueError):
-        UNet3DConditionModel(**cfg)
+    ref = _reference_outcome(i)
+    assert ref is not None and ref["type"] == "ValueError"
+    with pytest.raises(ValueError) as e:
+        UNet3DConditionModel(**BAD[i])
+    assert str(e.value) == ref["message"]
 
 
 def test_config_surface_and_parameters():
